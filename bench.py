@@ -9,7 +9,10 @@ Method (mirrors the reference's benchmarks/benchmark_inference.py:44-68): one in
 ``max_length = seq_len``, then one token per step through the public client API. ``value`` is device-timed over
 exactly K steps (CUDA events, barrier + synchronize on both sides, max over ranks) with tokens staying on the
 device; ``e2e`` repeats the K steps with, per step, the input token copied from pinned host memory and the sampled
-token read back to the host. Weights are random-init bf16 of the named architecture, prompts are synthetic ids.
+token read back to the host. Weights are random-init bf16 of the named architecture, prompts are synthetic ids. With
+N = 1 both come from fixed seeds, so the same arguments give the same inputs, and ``--dump-outputs DIR`` writes what the
+timed paths returned in their last step so that two builds can be compared output for output (the N > 1 paths draw
+their prompts from the global generator and do not dump).
 L2 hygiene: every decode step streams the full ~141 GB weight set (>> 126 MB L2), so inputs are larger than L2.
 """
 from __future__ import annotations
@@ -55,13 +58,25 @@ def main() -> None:
     ap.add_argument("--skip-selftests", action="store_true", help="N > 1: do not run the TP / pipeline numerics self-tests before the timed runs")
     ap.add_argument("--skip-pipeline", action="store_true", help="N > 1: do not append the pipeline-parallel record (same model as N stages)")
     ap.add_argument("--pp-chunk-tokens", type=int, default=256, help="positions per chunk of the pipelined prompt ingestion (pipeline record)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="N = 1: after the timed runs, write what each timed path returned in its last step "
+                    "as DIR/<name>.npy (token ids as float64, a fixed sample of prefill hidden-state rows as float32)")
     args = ap.parse_args()
     if args.impl == "reference":
         return reference_arm(args)
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.warmup < 3:
         args.warmup = 3
+    # generate() adds nothing once the session is full: make room for the prompt, the warm-up and both K-step loops
+    need = args.prompt_len + args.warmup + 2 * args.steps
+    if args.seq_len < need:
+        print(f"note: --seq-len raised from {args.seq_len} to {need} to hold the prompt, {args.warmup} warm-up and 2 x {args.steps} "
+              f"timed steps (decode runs at a longer KV length than requested)", file=sys.stderr)
+        args.seq_len = need
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1 or args.gpus > 1:
+        if args.dump_outputs:
+            ap.error("--dump-outputs is implemented for --gpus 1 only")
         from petals_b200.parallel.multi_gpu_bench import run_multi_gpu
 
         return run_multi_gpu(args)
@@ -95,13 +110,15 @@ def run_single_gpu(args) -> None:
     build_s = time.time() - t0
     K, W = args.steps, args.warmup
     vocab = model.config.vocab_size
-    prompt = torch.randint(0, vocab, (1, args.prompt_len), device=dev)
+    outputs = {}
+    prompt = torch.randint(0, vocab, (1, args.prompt_len), device=dev, generator=torch.Generator(dev).manual_seed(0))
     with torch.inference_mode(), model.inference_session(max_length=args.seq_len) as sess:
         prime_session(model, sess, prompt, W)  # prompt ingestion is not part of the single-stream metric, like the reference benchmark
         sampler = ClockSampler(0)
         sampler.start()
         ms, launches = device_timed_decode(model, sess, K)  # tokens never leave the GPU
         clocks = sampler.stop()
+        outputs["decode_token_ids"] = sess.output_ids.double().cpu().numpy()  # what the last timed generate() returned
         e2e_s, h2d, d2h = e2e_decode(model, sess, K, dev)  # pinned-host token in, sampled token out, every step
     value = K / (ms / 1e3)
     peaks = measured_peaks()
@@ -125,7 +142,7 @@ def run_single_gpu(args) -> None:
     }
     if not args.skip_prefill:
         try:
-            result["prefill"] = bench_prefill(model, args, peaks, spec, n_layers)
+            result["prefill"] = bench_prefill(model, args, peaks, spec, n_layers, outputs, "prefill")
         except Exception as e:  # noqa: BLE001 - the headline number must survive a failure of an appendix
             result["prefill"] = {"error": repr(e)[:200]}
     stage.shutdown()
@@ -136,13 +153,45 @@ def run_single_gpu(args) -> None:
 
             gc.collect()
             torch.cuda.empty_cache()
-            result["fp8_weights"] = bench_fp8_decode(args, path, n_layers, swarm, dev, K, W, spec, vocab, peaks)
+            result["fp8_weights"] = bench_fp8_decode(args, path, n_layers, swarm, dev, K, W, spec, vocab, peaks, outputs)
         except Exception as e:  # noqa: BLE001
             result["fp8_weights"] = {"error": repr(e)[:200]}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     print(json.dumps(result))
+    if args.dump_outputs:
+        expected = ["decode_token_ids"] + ([] if args.skip_prefill else ["prefill_hidden_rows"])
+        if not args.skip_fp8:
+            expected += ["fp8_decode_token_ids"] + ([] if args.skip_prefill else ["fp8_prefill_hidden_rows"])
+        missing = [n for n in expected if n not in outputs]
+        if missing:  # an appendix failed (its error is in the JSON line): the dump is incomplete
+            sys.exit(f"--dump-outputs: no output from {missing}")
 
 
-def bench_fp8_decode(args, path, n_layers, swarm, dev, K, W, spec, vocab, peaks) -> dict:
+def dump_outputs(directory: str, outputs: dict) -> None:
+    import numpy as np
+
+    total = sum(a.nbytes for a in outputs.values())
+    if total > 64 << 20:
+        raise ValueError(f"{total} bytes of outputs exceed the 64 MB dump budget")
+    for name, arr in outputs.items():
+        if arr.dtype not in (np.float32, np.float64):
+            raise TypeError(f"output {name} is {arr.dtype}, the dump holds float32 / float64 only")
+    os.makedirs(directory, exist_ok=True)
+    for name, arr in outputs.items():
+        np.save(os.path.join(directory, f"{name}.npy"), arr)
+
+
+def sample_rows(hidden, n: int = 256):
+    """A fixed, seeded sample of ``n`` rows of [..., H] hidden states, as float32 on the host (the full output is GBs)."""
+    import torch
+
+    flat = hidden.reshape(-1, hidden.shape[-1])
+    rows = torch.randperm(flat.shape[0], generator=torch.Generator().manual_seed(0))[:n].sort().values
+    return flat[rows.to(flat.device)].float().cpu().numpy()
+
+
+def bench_fp8_decode(args, path, n_layers, swarm, dev, K, W, spec, vocab, peaks, outputs) -> dict:
     """Same single-stream loop with the blocks served as block-scaled FP8 (MXFP8) weights — what `--quant_type fp8` serves in place
     of the reference's default NF4/INT8 (bitsandbytes has no sm_100 kernels). Compute stays bf16/fp32; reported next to, not
     instead of, the bf16 headline."""
@@ -156,10 +205,11 @@ def bench_fp8_decode(args, path, n_layers, swarm, dev, K, W, spec, vocab, peaks)
     try:
         model = random_client_model(path, swarm, dev)
         model.model.layers.sequence_manager.update(wait=True)
-        prompt = torch.randint(0, vocab, (1, 8), device=dev)
+        prompt = torch.randint(0, vocab, (1, 8), device=dev, generator=torch.Generator(dev).manual_seed(0))
         with torch.inference_mode(), model.inference_session(max_length=args.seq_len) as sess:
             prime_session(model, sess, prompt, W)
             ms, _ = device_timed_decode(model, sess, K)
+            outputs["fp8_decode_token_ids"] = sess.output_ids.double().cpu().numpy()
         value = K / (ms / 1e3)
         weight_bytes = spec.active_params() * n_layers * (1 + 1 / 32) + vocab * spec.hidden_size * 2
         rec = {"tokens_per_s": round(value, 3), "ms_per_step": round(ms / K, 4), "weight_bytes_per_token": int(weight_bytes),
@@ -167,7 +217,7 @@ def bench_fp8_decode(args, path, n_layers, swarm, dev, K, W, spec, vocab, peaks)
         if not args.skip_prefill:
             # prompt ingestion with BOTH operands in MXFP8 on the block-scaled tensor-core path (csrc/gemm_mxfp8.cu)
             try:
-                pf = bench_prefill(model, args, peaks, spec, n_layers)
+                pf = bench_prefill(model, args, peaks, spec, n_layers, outputs, "fp8_prefill")
                 pf["path"] = ("tcgen05.mma kind::mxf8f6f4.block_scale, activations quantised per 32 values (fused with the RMSNorm)"
                               if getattr(stage.stage.engine, "fp8_w8a8", False) else "weights dequantised per projection, bf16 tcgen05 GEMM")
                 rec["prefill"] = pf
@@ -178,13 +228,13 @@ def bench_fp8_decode(args, path, n_layers, swarm, dev, K, W, spec, vocab, peaks)
         stage.shutdown()
 
 
-def bench_prefill(model, args, peaks, spec, n_layers) -> dict:
+def bench_prefill(model, args, peaks, spec, n_layers, outputs, name) -> dict:
     """Parallel forward (benchmark_forward.py analogue): tokens/s = B*T / step time, no LM head."""
     import torch
 
     dev = "cuda:0"
     B, T = args.prefill_batch, args.prefill_seq
-    ids = torch.randint(0, model.config.vocab_size, (B, T), device=dev)
+    ids = torch.randint(0, model.config.vocab_size, (B, T), device=dev, generator=torch.Generator(dev).manual_seed(1))
     with torch.inference_mode():
         for _ in range(1):
             model.model(input_ids=ids)
@@ -192,9 +242,10 @@ def bench_prefill(model, args, peaks, spec, n_layers) -> dict:
         start, end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         start.record()
         for _ in range(args.prefill_steps):
-            model.model(input_ids=ids)
+            out = model.model(input_ids=ids)
         end.record()
         torch.cuda.synchronize()
+        outputs[f"{name}_hidden_rows"] = sample_rows(out.last_hidden_state)
     ms = start.elapsed_time(end) / args.prefill_steps
     flops = 2.0 * spec.active_params() * n_layers * B * T + 4.0 * n_layers * B * T * T * spec.num_heads * spec.head_dim / 2
     return {"tokens_per_s": round(B * T / (ms / 1e3), 1), "ms_per_step": round(ms, 2), "batch": B, "seq_len": T,

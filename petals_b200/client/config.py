@@ -40,12 +40,13 @@ class ClientConfig:
     use_server_to_server: bool = True  # let stage i hand its output to stage i+1 directly (fused NVLink hop / rpc_push)
     pipeline_chunk_tokens: int = 512  # a step of >= 2x this many tokens over >= 2 stages is ingested as a wavefront of chunks (0: never)
     # a client running on the stages' NVLink box may join their landing-ring fabric (run_server --fabric_address ...): its inputs reach the
-    # first stage and the last stage's outputs / gradients come back GPU to GPU. Needs a CUDA device for the client shell; collective:
-    # the fabric's world counts this client as one member.
+    # first stage and the last stage's outputs / gradients come back GPU to GPU (or through shared memory when the stages serve on CPU,
+    # see fabric_device); collective: the fabric's world counts this client as one member.
     fabric_address: Optional[str] = None  # "host:port" of the box's fabric rendezvous
     fabric_rank: Optional[int] = None
     fabric_world: Optional[int] = None
     fabric_max_tokens: int = 8192
+    fabric_device: Optional[str] = None  # where this member's landing rings live: None = the current CUDA device if any; "cpu" to join stages served on CPU
     show_route: Union[str, bool] = "inference"  # log the chosen chain: for inference sessions only, always (True) or never (False)
     max_pinged: int = 3  # how many candidate first-hop servers are pinged when a route is planned
     ping_timeout: float = 2

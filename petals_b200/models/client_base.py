@@ -150,7 +150,8 @@ class DistributedModelBase(nn.Module, PTuneMixin, FromPretrainedMixin):
         if getattr(config, "fabric_address", None):  # a client on the stages' box: become a member of their landing-ring fabric
             from petals_b200.parallel.fabric import join_fabric
 
-            join_fabric(config.fabric_address, config.fabric_rank, config.fabric_world, H, max_tokens=int(getattr(config, "fabric_max_tokens", 8192)))
+            join_fabric(config.fabric_address, config.fabric_rank, config.fabric_world, H, max_tokens=int(getattr(config, "fabric_max_tokens", 8192)),
+                        device=getattr(config, "fabric_device", None))
         self.layers = RemoteSequential(config, dht=dht)
         self.norm_weight = nn.Parameter(torch.ones(H), requires_grad=False)
         self.norm_bias = nn.Parameter(torch.zeros(H), requires_grad=False) if spec.norm == "layer" else None

@@ -288,13 +288,17 @@ class HostFabric:
             pass
 
 
-def init_fabric(hidden_size: int, max_tokens: int = 8192, group=None, host_dtype: torch.dtype = torch.float32, n_slots: int = 4):
-    """Collective over ``group``. Returns None when there is nothing to connect (single process)."""
+def init_fabric(hidden_size: int, max_tokens: int = 8192, group=None, host_dtype: torch.dtype = torch.float32, n_slots: int = 4,
+                cuda: Optional[bool] = None):
+    """Collective over ``group``. Returns None when there is nothing to connect (single process). ``cuda``: the landing rings live
+    in GPU memory (default: when a CUDA device is visible) or, for members that serve on the CPU, in host shared memory."""
     global _fabric
     if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) < 2:
         return None
+    if cuda is None:
+        cuda = torch.cuda.is_available()
     # the landing rings live at the same offsets of every member's heap: every member must size them identically
-    mine = (int(hidden_size), int(max_tokens), int(n_slots), bool(torch.cuda.is_available()))
+    mine = (int(hidden_size), int(max_tokens), int(n_slots), bool(cuda))
     everyone = [None] * dist.get_world_size(group)
     try:
         dist.all_gather_object(everyone, mine, group=group)
@@ -303,7 +307,7 @@ def init_fabric(hidden_size: int, max_tokens: int = 8192, group=None, host_dtype
         everyone = [mine]
     if any(other != mine for other in everyone):
         raise ValueError(f"the members of a fabric must agree on (hidden_size, max_tokens, n_slots, cuda): {everyone}")
-    if torch.cuda.is_available():
+    if cuda:
         _fabric = Fabric(hidden_size, max_tokens, group, n_slots=n_slots)
     else:
         _fabric = HostFabric(hidden_size, min(max_tokens, 1024), group, host_dtype, n_slots=n_slots)
@@ -332,15 +336,15 @@ def join_fabric(address: str, rank: int, world: int, hidden_size: int, *, device
     if _fabric is not None:
         return _fabric, False
     owns = False
+    device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device()) if torch.cuda.is_available() else torch.device("cpu")
+    cuda = device.type == "cuda"  # a member that serves on the CPU joins the shared-memory fabric, GPU or not
     if not dist.is_initialized():
-        device = torch.device(device) if device is not None else torch.device("cuda", torch.cuda.current_device()) if torch.cuda.is_available() else torch.device("cpu")
-        cuda = device.type == "cuda"
         if cuda:
             torch.cuda.set_device(device)
         dist.init_process_group(backend="cpu:gloo,cuda:nccl" if cuda else "gloo", init_method=f"tcp://{address}", rank=rank, world_size=world,
                                 **({"device_id": device} if cuda else {}))
         owns = True
-    fabric = init_fabric(hidden_size, max_tokens=max_tokens, host_dtype=host_dtype, n_slots=n_slots)
+    fabric = init_fabric(hidden_size, max_tokens=max_tokens, host_dtype=host_dtype, n_slots=n_slots, cuda=cuda)
     logger.info(f"Joined the NVLink fabric {str(getattr(fabric, 'fabric_id', '?'))[:8]} as member {rank} of {world} ({fabric.max_tokens} rows per landing slot)")
     return fabric, owns
 

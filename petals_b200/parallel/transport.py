@@ -16,6 +16,7 @@ src/petals/client/inference_session.py:198-207).
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 import errno
 import os
@@ -64,6 +65,23 @@ def to_multiaddr(address: str) -> str:
     return f"/{proto}/{host}/tcp/{port}"
 
 
+_SUN_PATH_MAX = 107  # bytes of a Unix socket path (sockaddr_un.sun_path holds 108 with the terminating NUL)
+
+
+@contextlib.contextmanager
+def _unix_name(path: str):
+    """A name that binds / connects to the Unix socket at ``path`` however deep its directory is (a rendezvous directory may live under
+    a long temp path): ``path`` itself when it fits, else the same file reached through a descriptor of its directory."""
+    if len(os.fsencode(path)) <= _SUN_PATH_MAX:
+        yield path
+        return
+    fd = os.open(os.path.dirname(path) or ".", os.O_PATH | os.O_DIRECTORY)
+    try:
+        yield f"/proc/self/fd/{fd}/{os.path.basename(path)}"
+    finally:
+        os.close(fd)
+
+
 def open_connection(address: str, connect_timeout: float, request_timeout: Optional[float]) -> socket.socket:
     kind, *rest = parse_address(address)
     if kind == "tcp":
@@ -72,7 +90,8 @@ def open_connection(address: str, connect_timeout: float, request_timeout: Optio
     else:
         s = socket.socket(socket.AF_UNIX, socket.SOCK_STREAM)
         s.settimeout(connect_timeout)
-        s.connect(rest[0])
+        with _unix_name(rest[0]) as name:
+            s.connect(name)
     s.settimeout(request_timeout)
     return s
 
@@ -318,7 +337,8 @@ class RpcServer:
             if os.path.exists(address):
                 os.unlink(address)
             self.socket_path = self.address = address
-            self._server = _ThreadedUnixServer(address, conn_class or _Conn)
+            with _unix_name(address) as name:
+                self._server = _ThreadedUnixServer(name, conn_class or _Conn)
         self._server.rpc_handler = handler  # type: ignore[attr-defined]
         self._server.open_conns, self._server.open_conns_lock = set(), threading.Lock()  # type: ignore[attr-defined]
         self._thread = threading.Thread(target=self._server.serve_forever, kwargs=dict(poll_interval=0.1), daemon=True)

@@ -10,12 +10,10 @@ NVLINK_PEER_GBS = 770.0  # measured peer-copy bandwidth per direction on this po
 
 def measured_peaks() -> dict:
     here = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    for path in (os.path.join(here, "MEASURED_PEAKS.json"), "/root/repo/MEASURED_PEAKS.json"):
-        try:
-            with open(path) as f:
-                d = json.load(f)
-            return dict(hbm_gbs=float(d["hbm_gbs"]), bf16_tflops=float(d["bf16_tflops"]),
-                        bf16_tflops_sustained=float(d.get("bf16_tflops_sustained", d["bf16_tflops"])), source="measured")
-        except Exception:
-            continue
-    return dict(_FALLBACK)
+    try:
+        with open(os.path.join(here, "MEASURED_PEAKS.json")) as f:
+            d = json.load(f)
+        return dict(hbm_gbs=float(d["hbm_gbs"]), bf16_tflops=float(d["bf16_tflops"]),
+                    bf16_tflops_sustained=float(d.get("bf16_tflops_sustained", d["bf16_tflops"])), source="measured")
+    except Exception:
+        return dict(_FALLBACK)

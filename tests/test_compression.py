@@ -160,6 +160,22 @@ def test_transport_default_is_exact(echo_server):
     assert torch.equal(out, x + 1)
 
 
+def test_unix_socket_in_a_deep_directory(tmp_path):
+    """A rendezvous directory may sit under a long temp path: a socket path longer than sun_path's 108 bytes still serves."""
+    deep = tmp_path / ("d" * 60) / ("e" * 60)
+    deep.mkdir(parents=True)
+    path = str(deep / "s.sock")
+    assert len(path) > 108
+    server = RpcServer(_EchoHandler(), path)
+    server.start()
+    try:
+        x = _hidden()
+        assert torch.equal(RemoteHandlerProxy(path).rpc_forward(["m.0"], x), x + 1)
+    finally:
+        server.shutdown()
+    assert not os.path.exists(path)
+
+
 def test_transport_server_default_and_per_request_override(echo_server):
     handler, path = echo_server
     x = _hidden(dtype=torch.float32)

@@ -91,7 +91,7 @@ def test_run_server_processes_join_a_fabric_and_serve_a_client_outside_it(member
     try:
         # member_client: this process joins the fabric as its third member (from_pretrained(..., fabric_address=...)): the last stage then
         # returns through the client's own landing ring and the client stores the output gradient into the last stage's ring
-        extra = dict(fabric_address=f"127.0.0.1:{port}", fabric_rank=2, fabric_world=3, fabric_max_tokens=256) if member_client else {}
+        extra = dict(fabric_address=f"127.0.0.1:{port}", fabric_rank=2, fabric_world=3, fabric_max_tokens=256, fabric_device="cpu") if member_client else {}
         model = AutoDistributedModelForCausalLM.from_pretrained(path, initial_peers=[rendezvous], max_retries=150, min_backoff=0.5, max_backoff=1.0, **extra)
         config = AutoDistributedConfig.from_pretrained(path)
         ids = torch.randint(0, config.vocab_size, (2, 9), generator=torch.Generator().manual_seed(0))
