@@ -339,7 +339,7 @@ __host__ __device__ constexpr uint32_t umma_idesc_e4m3(uint32_t M, uint32_t N) {
 // ---- host: launch with (optional) programmatic dependent launch ------------------------------------------------------
 // pb_pdl_enabled() reads PETALS_B200_PDL once (default on). Kernels launched through launch_pdl() MUST call pdl_wait()
 // before reading anything an earlier kernel of the stream produced.
-enum PdlKind : int { kPdlGemv = 1, kPdlRope = 2, kPdlAttn = 4, kPdlCombine = 8, kPdlGemvBigSmem = 16, kPdlGemvAuto = 32, kPdlGemvChain = 64 };
+enum PdlKind : int { kPdlGemv = 1, kPdlRope = 2, kPdlAttn = 4, kPdlCombine = 8, kPdlGemvBigSmem = 16, kPdlGemvAuto = 32 };
 inline int pdl_mask() {
   static const int mask = [] {
     const char* e = getenv("PETALS_B200_PDL");

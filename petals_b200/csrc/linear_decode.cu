@@ -74,8 +74,6 @@ struct LinearDecodeParams {
   int rope_T, rope_Hq, rope_Hkv, rope_D, rope_max_pages, rope_max_pos, rope_num_pages;
   int split_k;                                  // > 1: that many warps share one row pair, each streaming 1/split_k of K
   int pf_lines;                                 // 128-byte weight lines each warp prefetches into L2 before the prologue
-  int late_trigger;                             // 1: release the dependent kernel after the main loop instead of at entry
-  int wait_all_warps;                           // 1: every warp executes griddepcontrol.wait (default: warp 0 + barrier)
 };
 
 PB_DEVICE float gelu_tanh(float x) {
@@ -115,10 +113,11 @@ PB_DEVICE float block_sum(float v, float* red) {
 PB_DEVICE float rbf16(float x) { return __bfloat162float(__float2bfloat16_rn(x)); }
 
 // Warm L2 with the head of the first weight rows every warp will stream (weights are never written by a kernel, so this may
-// run before the producer of x has finished: behind a programmatic dependency, a peer-flag wait or a grid barrier).
+// run before the producer of x has finished: behind a programmatic dependency or a peer-flag wait).
 template <bool DUAL, bool ROPE>
-PB_DEVICE void gemv_prefetch(const LinearDecodeParams& p, int grid, int bid, int nwarps) {
+PB_DEVICE void gemv_prefetch(const LinearDecodeParams& p) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int grid = gridDim.x, bid = blockIdx.x, nwarps = blockDim.x >> 5;
   const int task0 = warp * grid + bid;
   if (warp < nwarps && task0 < (p.N >> 1) && p.pf_lines > 0) {
     constexpr int kRows = DUAL ? 4 : 2;
@@ -132,11 +131,10 @@ PB_DEVICE void gemv_prefetch(const LinearDecodeParams& p, int grid, int bid, int
   }
 }
 
-// One decode-shape linear layer executed by the whole CTA: `grid` CTAs cooperate, this one is number `bid`; warps >= nwarps
-// only take part in the prologue. M = tokens, DUAL = SwiGLU (two weight matrices), XSMEM = x staged in shared memory,
-// ROPE = fused RoPE + KV append epilogue. Called once by linear_decode_kernel and back to back by gemv_chain_kernel.
-template <int M, bool DUAL, bool XSMEM, bool ROPE, bool PIPE = false>
-PB_DEVICE void gemv_body(const LinearDecodeParams& p, uint8_t* smem_raw, int grid, int bid, int nwarps) {
+// One decode-shape linear layer; all CTAs of the grid cooperate. M = tokens, DUAL = SwiGLU (two weight matrices),
+// XSMEM = x staged in shared memory, ROPE = fused RoPE + KV append epilogue.
+template <int M, bool DUAL, bool XSMEM, bool ROPE>
+PB_DEVICE void gemv_body(const LinearDecodeParams& p, uint8_t* smem_raw) {
   __nv_bfloat16* xs = reinterpret_cast<__nv_bfloat16*>(smem_raw);
   __shared__ float red[32];
   __shared__ float stat[2 * M];
@@ -144,6 +142,7 @@ PB_DEVICE void gemv_body(const LinearDecodeParams& p, uint8_t* smem_raw, int gri
   const int K = p.K, N = p.N;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int tid = threadIdx.x, nthr = blockDim.x;
+  const int grid = gridDim.x, bid = blockIdx.x, nwarps = nthr >> 5;
 
   // ---- prologue ----------------------------------------------------------------------------
   if (p.wait_flag != nullptr) {
@@ -258,10 +257,7 @@ PB_DEVICE void gemv_body(const LinearDecodeParams& p, uint8_t* smem_raw, int gri
 
   // ---- main loop: each warp owns a pair of output columns ------------------------------------
   // A warp's work is the sequence of "slots" (task, it): U 16-byte loads per weight row of row pair `task` at K offset it*kstep.
-  //   !PIPE: load slot, multiply, next slot — 24 warps/SM hide the latency by interleaving.
-  //    PIPE: two slot buffers (512-thread CTAs, 128 registers): the next slot's loads — also across a task boundary — are issued
-  //          before the current slot is multiplied, so a warp always has loads in flight; short rows (tensor-parallel shards:
-  //          1-4 slots per task) no longer pay one exposed memory latency per task.
+  // Load slot, multiply, next slot: 24 warps/SM hide the latency by interleaving.
   constexpr int U = DUAL ? 2 : 4;  // 16-byte loads per weight row per slot (8 in flight per lane)
   const int ntasks = N >> 1;
   const int total_warps = grid * nwarps;
@@ -460,7 +456,7 @@ PB_DEVICE void gemv_body(const LinearDecodeParams& p, uint8_t* smem_raw, int gri
       for (int m = 0; m < M; ++m) a0[m] = a1[m] = b0[m] = b1[m] = 0.f;
       __syncthreads();
     }
-  } else if (!PIPE) {
+  } else {
     Slot s;
     for (; task < ntasks; task += total_warps) {
       for (int it = 0; it < nit; ++it) {
@@ -469,28 +465,8 @@ PB_DEVICE void gemv_body(const LinearDecodeParams& p, uint8_t* smem_raw, int gri
       }
       finish_task(task);
     }
-  } else {
-    Slot sa, sb;
-    int it = 0;
-    if (task < ntasks) load_slot(sa, task, 0);
-    while (task < ntasks) {
-      int t1 = task, i1 = it + 1;
-      if (i1 == nit) { i1 = 0; t1 += total_warps; }
-      if (t1 < ntasks) load_slot(sb, t1, i1);
-      compute_slot(sa, it);
-      if (it == nit - 1) finish_task(task);
-      task = t1; it = i1;
-      if (task >= ntasks) break;
-      int t2 = task, i2 = it + 1;
-      if (i2 == nit) { i2 = 0; t2 += total_warps; }
-      if (t2 < ntasks) load_slot(sa, t2, i2);
-      compute_slot(sb, it);
-      if (it == nit - 1) finish_task(task);
-      task = t2; it = i2;
-    }
   }
 
-  if (p.late_trigger && tid == 0) pdl_trigger();
   // ---- publish: every CTA fences its peer stores and checks in on a local counter; the last one to arrive
   // performs ONE release-increment per peer (so a consumer waits for `n_sources` per step, independent of grids).
   if (p.n_push > 0) {
@@ -508,110 +484,23 @@ PB_DEVICE void gemv_body(const LinearDecodeParams& p, uint8_t* smem_raw, int gri
   }
 }
 
-template <int M, bool DUAL, bool XSMEM, bool ROPE = false, bool PIPE = false>
-__global__ void __launch_bounds__((M <= 4 && !PIPE ? 768 : 512), 1) linear_decode_kernel(const LinearDecodeParams p) {
+template <int M, bool DUAL, bool XSMEM, bool ROPE = false>
+__global__ void __launch_bounds__((M <= 4 ? 768 : 512), 1) linear_decode_kernel(const LinearDecodeParams p) {
   extern __shared__ __align__(16) uint8_t smem_raw[];
   // ---- PDL pre-section: while the predecessor kernel drains (and while this kernel then waits for a peer flag and normalises x)
   // every warp pulls the head of its first weight rows into L2, so HBM keeps streaming through the bubble between two GEMVs
-  if (!p.late_trigger && threadIdx.x == 0) pdl_trigger();
-  gemv_prefetch<DUAL, ROPE>(p, gridDim.x, blockIdx.x, blockDim.x >> 5);
-  // one warp parks on the grid dependency, the rest of the CTA parks on the barrier behind it
-  if (p.wait_all_warps || (threadIdx.x >> 5) == 0) pdl_wait();
-  __syncthreads();
-  gemv_body<M, DUAL, XSMEM, ROPE, PIPE>(p, smem_raw, gridDim.x, blockIdx.x, blockDim.x >> 5);
-}
-
-// ---- a chain of dependent decode linears in ONE persistent launch ------------------------------------------------------------
-// O-projection -> gate/up (+SwiGLU) -> down [-> next block's QKV with RoPE/KV append]: four kernel boundaries per block become
-// grid barriers (or nothing at all where the consumer polls LL all-reduce payloads from every rank, itself included). At
-// tensor-parallel shard sizes a boundary costs about as much as streaming the weights; while a CTA waits at a barrier its warps
-// have already prefetched the next phase's first weight rows into L2.
-constexpr int kMaxChain = 4;
-struct GemvChainParams {
-  LinearDecodeParams ph[kMaxChain];
-  int n_phases;
-  int nwarps[kMaxChain];          // active warps per phase (tail-quantisation heuristic of the standalone launch)
-  int dual[kMaxChain], rope[kMaxChain];
-  int barrier_after[kMaxChain];   // 1: grid barrier between phase i and i+1; 0: data-flow synchronised (LL polling)
-  unsigned int* bar;              // {arrival count, generation} of THIS launch site, zero-initialised once
-  int n_barriers;
-};
-
-// Sense-reversing grid barrier on {arrival count, generation}: the last CTA to arrive resets the count and bumps the generation,
-// everyone else spins on the generation it read BEFORE arriving (it cannot change until this CTA has arrived too). Self-contained:
-// no step counter, any launch of the site works as long as all its CTAs are co-resident (grid <= #SMs, one CTA per SM).
-// `bar` points at 64 zero-initialised 32-bit words (two 128-byte lines).
-PB_DEVICE void grid_barrier(unsigned int* bar, int grid, int* error_flag) {
-  // bar[0] = arrival count, bar[32] = generation (separate 128-byte lines: pollers must not queue in front of the arrivals' atomics)
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    volatile unsigned int* gen_p = reinterpret_cast<volatile unsigned int*>(bar + 32);
-    const unsigned int gen = *gen_p;
-    __threadfence();
-    const unsigned int prev = atomicAdd(bar, 1u);
-    if (prev == static_cast<unsigned int>(grid) - 1u) {
-      *reinterpret_cast<volatile unsigned int*>(bar) = 0u;
-      __threadfence();
-      atomicAdd(bar + 32, 1u);
-    } else {
-      const uint64_t t0 = globaltimer_ns();
-      unsigned spins = 0;
-      while (*gen_p == gen) {
-        __nanosleep(40);
-        if ((++spins & 0x3ffu) == 0 && globaltimer_ns() - t0 > PB_FLAG_TIMEOUT_NS) {
-          if (error_flag != nullptr) atomicExch(error_flag, 1);
-          break;
-        }
-      }
-    }
-    __threadfence();
-  }
-  __syncthreads();
-}
-
-// The phases have FIXED roles by position (0: O-projection, 1: MLP input projection, 2: down projection, 3: next block's QKV with
-// RoPE/KV append), so every gemv_body below reads its parameters from a compile-time offset of the kernel's constant bank, exactly
-// like the standalone kernels do. (Indexing c.ph[] at run time — or passing the block by pointer to a non-inlined function — turns
-// those operands into register-held loads and made ptxas spill the weight buffers of the main loop: 25 % slower.)
-template <int M>
-__global__ void __launch_bounds__(768, 1) gemv_chain_kernel(const __grid_constant__ GemvChainParams c) {
-  extern __shared__ __align__(16) uint8_t smem_raw[];
-  const int grid = gridDim.x, bid = blockIdx.x;
   if (threadIdx.x == 0) pdl_trigger();
-  gemv_prefetch<false, false>(c.ph[0], grid, bid, c.nwarps[0]);
+  gemv_prefetch<DUAL, ROPE>(p);
+  // one warp parks on the grid dependency, the rest of the CTA parks on the barrier behind it
   if ((threadIdx.x >> 5) == 0) pdl_wait();
   __syncthreads();
-
-  // ---- phase 0: O-projection (+ residual / + LL push of the partial) ----
-  gemv_body<M, false, true, false>(c.ph[0], smem_raw, grid, bid, c.nwarps[0]);
-  // next phase's first weight rows -> L2 while we wait for the other CTAs (or for the peers' partial sums)
-  if (c.dual[1]) gemv_prefetch<true, false>(c.ph[1], grid, bid, c.nwarps[1]);
-  else gemv_prefetch<false, false>(c.ph[1], grid, bid, c.nwarps[1]);
-  if (c.barrier_after[0]) grid_barrier(c.bar, grid, c.ph[0].error_flag);
-  else __syncthreads();  // shared memory (x staging, reduction scratch) is reused by the next phase
-
-  // ---- phase 1: norm + gate/up (+SwiGLU) or up (+GELU) ----
-  if (c.dual[1]) gemv_body<M, true, true, false>(c.ph[1], smem_raw, grid, bid, c.nwarps[1]);
-  else gemv_body<M, false, true, false>(c.ph[1], smem_raw, grid, bid, c.nwarps[1]);
-  gemv_prefetch<false, false>(c.ph[2], grid, bid, c.nwarps[2]);
-  if (c.barrier_after[1]) grid_barrier(c.bar, grid, c.ph[1].error_flag);
-  else __syncthreads();
-
-  // ---- phase 2: down projection (+ residual / + LL push / + stage-hop push) ----
-  gemv_body<M, false, true, false>(c.ph[2], smem_raw, grid, bid, c.nwarps[2]);
-  if (c.n_phases > 3) {
-    gemv_prefetch<false, true>(c.ph[3], grid, bid, c.nwarps[3]);
-    if (c.barrier_after[2]) grid_barrier(c.bar, grid, c.ph[2].error_flag);
-    else __syncthreads();
-    // ---- phase 3: the next block's norm + QKV projection with RoPE + KV append ----
-    gemv_body<M, false, true, true>(c.ph[3], smem_raw, grid, bid, c.nwarps[3]);
-  }
+  gemv_body<M, DUAL, XSMEM, ROPE>(p, smem_raw);
 }
 
-template <int M, bool DUAL, bool XSMEM, bool ROPE = false, bool PIPE = false>
+template <int M, bool DUAL, bool XSMEM, bool ROPE = false>
 static cudaError_t launch_one(const LinearDecodeParams& p, int grid, int block, size_t smem,
                               cudaStream_t stream) {
-  auto kern = linear_decode_kernel<M, DUAL, XSMEM, ROPE, PIPE>;
+  auto kern = linear_decode_kernel<M, DUAL, XSMEM, ROPE>;
   if (smem > 32 * 1024) {  // static shared memory counts against the 48 KB default too
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          static_cast<int>(smem));
@@ -628,13 +517,7 @@ static cudaError_t launch_one(const LinearDecodeParams& p, int grid, int block, 
 
 template <int M>
 static cudaError_t launch_m(const LinearDecodeParams& p, bool dual, bool xsmem, int grid, int block,
-                            size_t smem, cudaStream_t s, bool pipe = false) {
-  if constexpr (M <= 2) {
-    if (pipe && xsmem) {  // software-pipelined main loop (512-thread CTAs)
-      if (p.rope_q_out != nullptr) return launch_one<M, false, true, true, true>(p, grid, block, smem, s);
-      return dual ? launch_one<M, true, true, false, true>(p, grid, block, smem, s) : launch_one<M, false, true, false, true>(p, grid, block, smem, s);
-    }
-  }
+                            size_t smem, cudaStream_t s) {
   if (p.rope_q_out != nullptr) return launch_one<M, false, true, true>(p, grid, block, smem, s);  // validated: !dual && xsmem
   if (dual) return xsmem ? launch_one<M, true, true>(p, grid, block, smem, s)
                          : launch_one<M, true, false>(p, grid, block, smem, s);
@@ -649,14 +532,7 @@ static cudaError_t launch_m(const LinearDecodeParams& p, bool dual, bool xsmem, 
 // ------------------------------------------------------------------------------------------------
 namespace pb {
 
-// software-pipelined main loop for M <= 2 (PETALS_B200_GEMV_PIPE, or pb_set_gemv_pipe at run time)
-static int g_gemv_pipe = -1;
-static int gemv_pipe_mode() {
-  if (g_gemv_pipe < 0) { const char* e = getenv("PETALS_B200_GEMV_PIPE"); g_gemv_pipe = e ? atoi(e) : 0; }
-  return g_gemv_pipe;
-}
-
-struct GemvGeom { bool dual, xsmem, pipe; size_t smem; int grid, best_w; };
+struct GemvGeom { bool dual, xsmem; size_t smem; int grid, best_w; };
 
 // Validate one linear's arguments, translate them into kernel parameters and pick its launch geometry.
 static int gemv_fill(const PbLinearDecodeArgs* a, LinearDecodeParams& p, GemvGeom& g) {
@@ -715,13 +591,9 @@ static int gemv_fill(const PbLinearDecodeArgs* a, LinearDecodeParams& p, GemvGeo
   {
     static const int env_pf = [] { const char* e = getenv("PETALS_B200_PF_LINES"); return e ? atoi(e) : -1; }();
     static const int env_pf_wait = [] { const char* e = getenv("PETALS_B200_PF_LINES_WAIT"); return e ? atoi(e) : -1; }();
-    static const int env_late = [] { const char* e = getenv("PETALS_B200_PDL_LATE"); return e ? atoi(e) : 0; }();
     // a kernel that will spin on a peer flag can hide a deep prefetch behind the wait; one that starts right away cannot
     p.pf_lines = (a->wait_flag != nullptr || a->n_ll_parts > 0) ? (env_pf_wait >= 0 ? env_pf_wait : 64) : (env_pf >= 0 ? env_pf : 16);
     if (p.pf_lines > 0 && p.pf_lines < 4) p.pf_lines = 4;
-    p.late_trigger = env_late;
-    static const int env_allw = [] { const char* e = getenv("PETALS_B200_PDL_WAIT_ALL"); return e ? atoi(e) : 0; }();
-    p.wait_all_warps = env_allw;
   }
   p.done_counter = static_cast<unsigned int*>(a->done_counter);
   if (a->n_push > 0 && p.done_counter == nullptr) return PB_ERR_SHAPE;
@@ -738,8 +610,7 @@ static int gemv_fill(const PbLinearDecodeArgs* a, LinearDecodeParams& p, GemvGeo
   // was requested (flag accounting across ranks needs identical CTA counts) honour it.
   const int sms = a->fixed_grid > 0 ? a->fixed_grid : (a->num_sms > 0 ? a->num_sms : 148);
   const int ntasks = a->N / 2;
-  const bool pipe = gemv_pipe_mode() != 0 && a->M <= 2 && xsmem;
-  const int max_w = (a->M <= 4 && !pipe) ? 24 : 16;
+  const int max_w = a->M <= 4 ? 24 : 16;
   int best_w = max_w;
   double best_eff = -1.0;
   for (int w = max_w; w >= max_w / 2; --w) {
@@ -750,13 +621,13 @@ static int gemv_fill(const PbLinearDecodeArgs* a, LinearDecodeParams& p, GemvGeo
   }
   p.split_k = 1;
   static const int env_splitk = [] { const char* e = getenv("PETALS_B200_GEMV_SPLITK"); return e ? atoi(e) : 1; }();
-  if (env_splitk && !pipe && xsmem && a->M <= 4 && a->fixed_grid <= 0 && ntasks < sms * 12 && a->K >= 2048) {
+  if (env_splitk && xsmem && a->M <= 4 && a->fixed_grid <= 0 && ntasks < sms * 12 && a->K >= 2048) {
     // few output columns: spread the row pairs over ALL SMs and let 4 (or 2) warps share each pair along K
     const int groups = (ntasks + sms - 1) / sms;
     const int S = groups * 4 <= 24 ? 4 : (groups * 2 <= 24 ? 2 : 1);
     if (S > 1) {
       p.split_k = S;
-      g.dual = a->act == 1; g.xsmem = xsmem; g.pipe = false; g.smem = smem; g.grid = sms; g.best_w = groups * S;
+      g.dual = a->act == 1; g.xsmem = xsmem; g.smem = smem; g.grid = sms; g.best_w = groups * S;
       return PB_OK;
     }
   }
@@ -767,13 +638,11 @@ static int gemv_fill(const PbLinearDecodeArgs* a, LinearDecodeParams& p, GemvGeo
     if (grid > sms) grid = sms;
   }
   if (a->fixed_grid > 0) grid = a->fixed_grid;
-  g.dual = dual; g.xsmem = xsmem; g.pipe = pipe; g.smem = smem; g.grid = grid; g.best_w = best_w;
+  g.dual = dual; g.xsmem = xsmem; g.smem = smem; g.grid = grid; g.best_w = best_w;
   return PB_OK;
 }
 
 }  // namespace pb
-
-extern "C" int pb_set_gemv_pipe(int on) { pb::g_gemv_pipe = on ? 1 : 0; return PB_OK; }
 
 extern "C" int pb_linear_decode(const PbLinearDecodeArgs* a, void* stream) {
   using namespace pb;
@@ -788,14 +657,14 @@ extern "C" int pb_linear_decode(const PbLinearDecodeArgs* a, void* stream) {
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   cudaError_t e = cudaSuccess;
   switch (a->M) {
-    case 1: e = launch_m<1>(p, dual, xsmem, grid, block, smem, s, g.pipe); break;
-    case 2: e = launch_m<2>(p, dual, xsmem, grid, block, smem, s, g.pipe); break;
-    case 3: e = launch_m<3>(p, dual, xsmem, grid, block, smem, s, g.pipe); break;
-    case 4: e = launch_m<4>(p, dual, xsmem, grid, block, smem, s, g.pipe); break;
-    case 5: e = launch_m<5>(p, dual, xsmem, grid, block, smem, s, g.pipe); break;
-    case 6: e = launch_m<6>(p, dual, xsmem, grid, block, smem, s, g.pipe); break;
-    case 7: e = launch_m<7>(p, dual, xsmem, grid, block, smem, s, g.pipe); break;
-    case 8: e = launch_m<8>(p, dual, xsmem, grid, block, smem, s, g.pipe); break;
+    case 1: e = launch_m<1>(p, dual, xsmem, grid, block, smem, s); break;
+    case 2: e = launch_m<2>(p, dual, xsmem, grid, block, smem, s); break;
+    case 3: e = launch_m<3>(p, dual, xsmem, grid, block, smem, s); break;
+    case 4: e = launch_m<4>(p, dual, xsmem, grid, block, smem, s); break;
+    case 5: e = launch_m<5>(p, dual, xsmem, grid, block, smem, s); break;
+    case 6: e = launch_m<6>(p, dual, xsmem, grid, block, smem, s); break;
+    case 7: e = launch_m<7>(p, dual, xsmem, grid, block, smem, s); break;
+    case 8: e = launch_m<8>(p, dual, xsmem, grid, block, smem, s); break;
   }
   if (e != cudaSuccess) {
     cudaGetLastError();
@@ -805,65 +674,4 @@ extern "C" int pb_linear_decode(const PbLinearDecodeArgs* a, void* stream) {
     return PB_ERR_CUDA;
   }
   return a->out_grid ? (*(a->out_grid) = grid, PB_OK) : PB_OK;
-}
-
-// A chain of dependent decode linears in one persistent launch (see gemv_chain_kernel). `phases[i]` are ordinary linear_decode
-// argument blocks; `barrier_after[i]` says whether phase i+1 may only start once EVERY CTA finished phase i (a grid barrier) or
-// is synchronised by data flow (it polls LL all-reduce payloads). `bar` points at two zero-initialised 32-bit words
-// {arrival count, generation} owned by this launch site.
-extern "C" int pb_gemv_chain(const PbLinearDecodeArgs* const* phases, int n_phases, const int* barrier_after, void* bar, void* stream) {
-  using namespace pb;
-  if (n_phases < 3 || n_phases > kMaxChain) return PB_ERR_SHAPE;  // O-proj, MLP-in, down [, next QKV]
-  GemvChainParams c{};
-  c.n_phases = n_phases;
-  const int M = phases[0]->M;
-  if (M < 1 || M > 4) return PB_ERR_SHAPE;  // 768-thread CTAs: the register budget of the M <= 4 variants
-  const int sms = phases[0]->num_sms > 0 ? phases[0]->num_sms : 148;
-  size_t smem = 0;
-  for (int i = 0; i < n_phases; ++i) {
-    GemvGeom g;
-    const int rc = gemv_fill(phases[i], c.ph[i], g);
-    if (rc != PB_OK) return rc;
-    if (phases[i]->M != M || !g.xsmem || phases[i]->fixed_grid > 0) return PB_ERR_SHAPE;
-    c.ph[i].split_k = 1;  // the chain distributes row pairs itself (nwarps below)
-    c.dual[i] = g.dual ? 1 : 0;
-    c.rope[i] = c.ph[i].rope_q_out != nullptr ? 1 : 0;
-    if ((i != 1 && c.dual[i]) || c.rope[i] != (i == 3 ? 1 : 0)) return PB_ERR_SHAPE;  // fixed roles by position
-    // all phases share the full grid; a phase with few output columns keeps its tasks spread over all SMs with fewer warps
-    const int ntasks = phases[i]->N / 2;
-    c.nwarps[i] = (ntasks < sms * g.best_w || g.grid != sms) ? (ntasks + sms - 1) / sms : g.best_w;
-    if (c.nwarps[i] < 1) c.nwarps[i] = 1;
-    if (c.nwarps[i] > 24) c.nwarps[i] = 24;
-    if (g.smem > smem) smem = g.smem;
-    c.barrier_after[i] = (i + 1 < n_phases && barrier_after != nullptr && barrier_after[i]) ? 1 : 0;
-    c.n_barriers += c.barrier_after[i];
-    // inside the chain a phase never waits on a programmatic dependency of its own; deep prefetch is issued by the chain kernel
-    static const int chain_pf = [] { const char* e = getenv("PETALS_B200_CHAIN_PF"); return e ? atoi(e) : 16; }();
-    c.ph[i].pf_lines = i == 0 ? c.ph[i].pf_lines : (chain_pf > 0 && chain_pf < 4 ? 4 : chain_pf);
-  }
-  if (c.n_barriers > 0 && bar == nullptr) return PB_ERR_SHAPE;
-  c.bar = static_cast<unsigned int*>(bar);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  cudaError_t e = cudaSuccess;
-  auto launch = [&](auto kern) {
-    if (smem > 32 * 1024) {
-      const cudaError_t ea = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
-      if (ea != cudaSuccess) return ea;
-    }
-    return launch_pdl(kPdlGemvChain, kern, dim3(sms), dim3(768), smem, s, c);
-  };
-  switch (M) {
-    case 1: e = launch(gemv_chain_kernel<1>); break;
-    case 2: e = launch(gemv_chain_kernel<2>); break;
-    case 3: e = launch(gemv_chain_kernel<3>); break;
-    case 4: e = launch(gemv_chain_kernel<4>); break;
-  }
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    char what[160];
-    snprintf(what, sizeof(what), "gemv_chain M=%d phases=%d smem=%zu: %s", M, n_phases, smem, cudaGetErrorString(e));
-    pb_set_error(what);
-    return PB_ERR_CUDA;
-  }
-  return PB_OK;
 }

@@ -34,11 +34,8 @@ typedef struct {
   int rope_num_pages;           // pages in rope_k_pool / rope_v_pool: a table entry outside [0, num_pages) raises error flag 2
 } PbLinearDecodeArgs;
 int pb_linear_decode(const PbLinearDecodeArgs* a, void* stream);
-int pb_set_gemv_pipe(int on);
 // 2..8 rows on the tensor cores (mma.sync m16n8k16, tokens as the N dimension); scratch: fp32 [2*N*8] zeros, counters: u32 [N/16] zeros
-int pb_linear_decode_mma(const PbLinearDecodeArgs* a, void* scratch, void* counters, void* stream);  // M <= 2: software-pipelined main loop (512-thread CTAs, loads of the next slot in flight during the math)
-// up to 4 dependent decode linears in one persistent launch (grid barriers or LL data-flow between phases; linear_decode.cu)
-int pb_gemv_chain(const PbLinearDecodeArgs* const* phases, int n_phases, const int* barrier_after, void* bar, void* stream);
+int pb_linear_decode_mma(const PbLinearDecodeArgs* a, void* scratch, void* counters, void* stream);
 
 // ---- decode-shape linear over block-scaled FP8 weights (linear_decode_fp8.cu) ---------------------------
 typedef struct {

@@ -157,31 +157,6 @@ def _skinny_buffers(device: torch.device, N: int):
     return have[0], have[1]
 
 
-def set_gemv_pipe(on: bool) -> None:
-    """Select the software-pipelined decode-linear main loop (M <= 2). Default: env ``PETALS_B200_GEMV_PIPE`` (off)."""
-    native.lib().pb_set_gemv_pipe(int(bool(on)))
-
-
-def gemv_chain(phases: Sequence[dict], barrier_after: Sequence[bool], bar: Optional[torch.Tensor]) -> list:
-    """Run up to four dependent decode linears (O-projection -> gate/up -> down -> next block's QKV) as ONE persistent kernel.
-
-    ``phases`` are keyword dicts of :func:`linear_decode` (with ``x`` and ``w``); ``barrier_after[i]`` puts a grid barrier between
-    phase i and i+1 (omit it where phase i+1 polls LL all-reduce payloads instead). ``bar``: 64 zero-initialised int32 words
-    (arrival count and generation on separate 128-byte lines) owned by this launch site. Returns the phases' result tensors."""
-    n = len(phases)
-    arg_blocks, results, keep = [], [], []
-    for ph in phases:
-        kw = dict(ph)
-        a, r, k = _linear_decode_args(kw.pop("x"), kw.pop("w"), **kw)
-        arg_blocks.append(a)
-        results.append(r)
-        keep.append(k)
-    arr = (C.POINTER(LinearDecodeArgs) * n)(*[C.pointer(a) for a in arg_blocks])
-    bars = (C.c_int * n)(*[int(bool(b)) for b in list(barrier_after) + [False] * (n - len(barrier_after))])
-    check(native.lib().pb_gemv_chain(arr, n, bars, ptr(bar), stream_ptr()), "gemv_chain")
-    return results
-
-
 def linear_decode_fp8(x: torch.Tensor, w_q: torch.Tensor, w_scale: torch.Tensor, *, w2_q: Optional[torch.Tensor] = None,
                       w2_scale: Optional[torch.Tensor] = None, bias=None, bias2=None, residual=None, norm_weight=None, norm_bias=None,
                       norm_kind: int = NORM_NONE, eps: float = 1e-6, act: int = ACT_NONE, out: Optional[torch.Tensor] = None) -> torch.Tensor:

@@ -150,12 +150,8 @@ def _declare(lib: C.CDLL) -> None:
         getattr(lib, name).restype = ci
     lib.pb_linear_decode.argtypes = [C.POINTER(LinearDecodeArgs), vp]
     lib.pb_gemm_bf16.argtypes = [C.POINTER(GemmArgs), vp]
-    lib.pb_gemv_chain.argtypes = [C.POINTER(C.POINTER(LinearDecodeArgs)), ci, C.POINTER(C.c_int), vp, vp]
-    lib.pb_gemv_chain.restype = ci
     lib.pb_linear_decode_mma.argtypes = [C.POINTER(LinearDecodeArgs), vp, vp, vp]
     lib.pb_linear_decode_mma.restype = ci
-    lib.pb_set_gemv_pipe.argtypes = [ci]
-    lib.pb_set_gemv_pipe.restype = ci
     lib.pb_linear_decode_fp8.argtypes = [C.POINTER(LinearFp8Args), vp]
     lib.pb_linear_decode_fp8.restype = ci
     lib.pb_dequant_mxfp8.argtypes = [vp, vp, vp, cl, vp]

@@ -184,8 +184,6 @@ class TPDecodeEngine:
         self.err = torch.zeros(1, dtype=torch.int32, device=dev)
         self.done_counter = torch.zeros(1, dtype=torch.int32, device=dev)
         self.fuse_rope = os.environ.get("PETALS_B200_FUSE_ROPE", "1") != "0"
-        self.use_chain = os.environ.get("PETALS_B200_CHAIN", "0") != "0"
-        self._chain_bar = torch.zeros(max(1, len(self.shards)), 64, dtype=torch.int32, device=dev)  # grid-barrier words per block
         self._split_ctr = torch.zeros(1024, dtype=torch.int32, device=dev)  # split-KV arrival counters (self-resetting)
         self._moe_bufs: Dict[object, torch.Tensor] = {}  # sparse-MoE scratch (ops/functional.py: moe_decode / moe_prefill)
         self.pos_static = torch.zeros(1, dtype=torch.int32, device=dev)
@@ -263,7 +261,6 @@ class TPDecodeEngine:
         ll_mlp_in = [self.heap.addr(me, self.off_ll_mlp + r * self.ll_slot_bytes) for r in range(R)]
         ll_attn_out = [self.heap.addr(r, self.off_ll_attn + me * self.ll_slot_bytes) for r in range(R)]
         ll_mlp_out = [self.heap.addr(r, self.off_ll_mlp + me * self.ll_slot_bytes) for r in range(R)]
-        chain = self.use_chain and ll and self.fuse_rope and M <= 4
         split_ctr = self._split_ctr if splits > 1 and B * ls.num_kv_heads <= 1024 else None
 
         def k1_kwargs(l: int, cur, nxt):
@@ -337,17 +334,11 @@ class TPDecodeEngine:
             else:
                 k4 = dict(x=act, w=w["w_down"], store_local=False, push_out=[self.parts(self.off_parts_mlp, r, me) for r in range(R)],
                           push_flag=[self.flag_mlp(r, l) for r in range(R)], done_counter=ctr, error_flag=err)
-            phases = [k2, k3, k4]
+            for kw in (k2, k3, k4):
+                launch(kw)
             if l + 1 < L:
                 kw1, cur, nxt = k1_kwargs(l + 1, cur, nxt)
-                phases.append(kw1)
-            if chain:
-                # ONE persistent launch: K2 -> K3 are synchronised by the LL payloads K3 polls (from every rank, this one included),
-                # K3 -> K4 by a grid barrier (every CTA needs the whole activation vector), K4 -> next K1 by LL polling again
-                Fn.gemv_chain(phases, [False, True, False][: len(phases) - 1], self._chain_bar[l])
-            else:
-                for kw in phases:
-                    launch(kw)
+                launch(kw1)
         if final_reduce:
             parts = ptr_array(mlp_parts)
             native.check(native.lib().pb_reduce_parts(cur.data_ptr(), parts, R, self.flag_mlp(me, self.n_blocks - 1), R, ep_f, self.out.data_ptr(),
@@ -555,19 +546,6 @@ class TPDecodeEngine:
             Fn.linear_decode(x, w["w_up"], act=self.act, norm_weight=w["ln2_w"], norm_bias=w.get("ln2_b"), norm_kind=self.norm_kind,
                              eps=s.norm_eps, out=act, parts=[scratch], x_out=self._buf("h_b", M, H))
         Fn.linear_decode(act, w["w_down"], out=scratch)
-        if self.use_chain and self.use_ll and self.fuse_rope and M <= 4:
-            # the persistent chain kernel (same four phases, local buffers only)
-            pools = self.cache.layer_pools(0)
-            mlp = (dict(w=w["w_gate"], w2=w["w_up"], act=Fn.ACT_SWIGLU) if s.mlp == "swiglu" else dict(w=w["w_up"], act=self.act))
-            Fn.gemv_chain([
-                dict(x=attn, w=w["wo"], out=scratch),
-                dict(x=x, norm_weight=w["ln2_w"], norm_bias=w.get("ln2_b"), norm_kind=self.norm_kind, eps=s.norm_eps, out=act, **mlp),
-                dict(x=act, w=w["w_down"], out=scratch),
-                dict(x=x, w=w["wqkv"], norm_weight=w["ln1_w"], norm_bias=w.get("ln1_b"), norm_kind=self.norm_kind, eps=s.norm_eps,
-                     error_flag=self.err.data_ptr(),
-                     rope=dict(q_out=q_buf, k_pool=pools[0], v_pool=pools[1], block_table=table, pos_ptr=self.pos_static.data_ptr(), cos=self.cos,
-                               sin=self.sin, T=T, Hq=ls.num_heads, Hkv=ls.num_kv_heads, D=ls.head_dim)),
-            ], [True, True, True], self._chain_bar[0])
         torch.cuda.synchronize(self.device)
 
     # ---- session bookkeeping (identical on every rank) ---------------------------------------------------------------------

@@ -99,9 +99,6 @@ class StageEngine:
         self.pos_static = torch.zeros(1, dtype=torch.int32, device=self.device)
         self.err_flag = torch.zeros(1, dtype=torch.int32, device=self.device)
         self.fuse_rope = os.environ.get("PETALS_B200_FUSE_ROPE", "1") != "0"
-        # O-proj -> gate/up -> down -> next block's QKV as one persistent launch per block (grid barriers instead of kernel boundaries)
-        self.use_chain = os.environ.get("PETALS_B200_CHAIN", "0") != "0"
-        self._chain_bar = torch.zeros(max(1, len(self.blocks)), 64, dtype=torch.int32, device=self.device)  # {count, generation} per block
         # single-token steps of Llama-style spans as ONE persistent data-flow kernel (csrc/decode_span.cu): weights stream through
         # a shared-memory ring across what used to be kernel boundaries, phases are ordered by tagged data instead of launches
         self.use_span_kernel = os.environ.get("PETALS_B200_SPAN_KERNEL", "1") != "0" and self._span_kernel_ok()
@@ -458,47 +455,6 @@ class StageEngine:
             self._dev_pos = session.position
         return table
 
-    def _chain_ok(self, M: int, lo: int, hi: int, prompts) -> bool:
-        s = self.spec
-        return (self.use_chain and self._adapter is None and self.fuse_rope and M <= 4 and self.fp8 is None and prompts is None and s.mlp in ("swiglu", "gelu")
-                and not s.parallel_attn and not s.qkv_interleaved and not s.post_ln_residual
-                and all(self.blocks[i]._p("bqkv") is None for i in range(lo, hi)))
-
-    def _qkv_rope_kwargs(self, x: torch.Tensor, slot: int, M: int, T: int, table, pos_ptr, pools) -> dict:
-        """Arguments of the QKV projection with the fused RoPE + KV-append epilogue (standalone launch or last phase of a chain)."""
-        s, w = self.spec, self.blocks[slot]
-        return dict(x=x, w=w.wqkv, norm_weight=w.ln1_w, norm_bias=w._p("ln1_b"), norm_kind=self.norm_kind, eps=s.norm_eps,
-                    error_flag=self.err_flag.data_ptr(),
-                    rope=dict(q_out=self._buf("q", M, s.num_heads * s.head_dim), k_pool=pools[0], v_pool=pools[1], block_table=table,
-                              pos_ptr=pos_ptr, cos=self.cos, sin=self.sin, T=T, Hq=s.num_heads, Hkv=s.num_kv_heads, D=s.head_dim))
-
-    def _run_span_chain(self, x: torch.Tensor, B: int, T: int, lo: int, hi: int, table, pos_ptr, pools_of, splits: int,
-                        hop: Optional[tuple] = None) -> torch.Tensor:
-        """Decode step of blocks [lo, hi) with 2 launches per block: split-KV attention, then ONE persistent kernel running
-        O-projection(+residual) -> norm + gate/up (+SwiGLU) -> down(+residual) -> the next block's norm + QKV (+RoPE, KV append)
-        with grid barriers in place of kernel boundaries."""
-        s = self.spec
-        M, eps = B * T, s.norm_eps
-        h1 = self._buf("h_alt", M, s.hidden_size)
-        act = self._buf("act", M, s.intermediate_size)
-        kw0 = self._qkv_rope_kwargs(x, lo, M, T, table, pos_ptr, pools_of(lo))
-        Fn.linear_decode(kw0.pop("x"), kw0.pop("w"), **kw0)
-        for slot in range(lo, hi):
-            w = self.blocks[slot]
-            attn = self._attention(None, slot, B, T, table, pos_ptr, pools_of(slot), splits, "")
-            phases = [dict(x=attn, w=w.wo, bias=w._p("bo"), residual=x, out=h1)]
-            mlp = dict(x=h1, norm_weight=w.ln2_w, norm_bias=w._p("ln2_b"), norm_kind=self.norm_kind, eps=eps, out=act)
-            if s.mlp == "swiglu":
-                phases.append(dict(w=w.w_gate, w2=w.w_up, act=Fn.ACT_SWIGLU, **mlp))
-            else:
-                phases.append(dict(w=w.w_up, bias=w._p("b_up"), act=self.act, **mlp))
-            push = self._push_kwargs(hop) if slot == hi - 1 else {}
-            phases.append(dict(x=act, w=w.w_down, bias=w._p("b_down"), residual=h1, out=x, **push))
-            if slot + 1 < hi:
-                phases.append(self._qkv_rope_kwargs(x, slot + 1, M, T, table, pos_ptr, pools_of(slot + 1)))
-            Fn.gemv_chain(phases, [True] * (len(phases) - 1), self._chain_bar[slot])
-        return x
-
     def _run_span(self, x: torch.Tensor, B: int, T: int, lo: int, hi: int, table, pos_ptr, pools_of, prompts, decode: bool, splits: int,
                   hop: Optional[tuple] = None) -> torch.Tensor:
         M = B * T
@@ -506,8 +462,6 @@ class StageEngine:
                 and (self._adapter is None or self.lora_mode == "merged")):
             out = self._buf("h_alt", M, self.spec.hidden_size)
             return Fn.decode_span(self._span_kernel_plan(), x, out, table, pos_ptr, self.cos, self.sin, lo=lo, hi=hi)
-        if decode and self._chain_ok(M, lo, hi, prompts) and (hop is None or self.spec.mlp != "moe"):
-            return self._run_span_chain(x, B, T, lo, hi, table, pos_ptr, pools_of, splits, hop)
         other = self._buf("h_alt", M, self.spec.hidden_size) if decode else None
         cur = x
         for slot in range(lo, hi):

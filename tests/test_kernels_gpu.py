@@ -506,76 +506,6 @@ def test_linear_decode_fp8_activation_outliers():
         assert err < 2e-2, f"row {m}: {err}"
 
 
-@pytest.mark.parametrize("M", [1, 2, 4])
-def test_gemv_chain_matches_separate_launches(M):
-    """O-proj(+residual) -> norm + gate/up SwiGLU -> down(+residual) -> next block's norm + QKV with RoPE/KV append as ONE persistent
-    launch with grid barriers == the same four linears launched one by one (bit for bit), twice (barrier words are reusable)."""
-    torch.manual_seed(41)
-    H, I, D, Hq, Hkv, T = 1024, 2816, 64, 8, 2, 1
-    B = M // T
-    xres, attn = _rand(M, H), _rand(M, Hq * D)
-    wo, wg, wu, wd = _rand(H, Hq * D, scale=0.03), _rand(I, H, scale=0.03), _rand(I, H, scale=0.03), _rand(H, I, scale=0.02)
-    wqkv = _rand((Hq + 2 * Hkv) * D, H, scale=0.03)
-    ln2, ln1n = _rand(H) * 0.1 + 1, _rand(H) * 0.1 + 1
-    cos, sin = Fn.rope_tables(D, 512, theta=10000.0, device=DEV)
-    pos = torch.full((1,), 37, dtype=torch.int32, device=DEV)
-    kp_a, vp_a, table = _paged_setup(B, 128, Hkv, D, seed=7)
-    kp_b, vp_b = kp_a.clone(), vp_a.clone()
-
-    def run(chain: bool, kp, vp):
-        x = xres.clone()
-        h1, act, q = torch.empty(M, H, device=DEV, dtype=torch.bfloat16), torch.empty(M, I, device=DEV, dtype=torch.bfloat16), torch.empty(M, Hq * D, device=DEV, dtype=torch.bfloat16)
-        phases = [
-            dict(x=attn, w=wo, residual=x, out=h1),
-            dict(x=h1, w=wg, w2=wu, act=Fn.ACT_SWIGLU, norm_weight=ln2, norm_kind=Fn.NORM_RMS, eps=1e-5, out=act),
-            dict(x=act, w=wd, residual=h1, out=x),
-            dict(x=x, w=wqkv, norm_weight=ln1n, norm_kind=Fn.NORM_RMS, eps=1e-5,
-                 rope=dict(q_out=q, k_pool=kp, v_pool=vp, block_table=table, pos_ptr=pos.data_ptr(), cos=cos, sin=sin, T=T, Hq=Hq, Hkv=Hkv, D=D)),
-        ]
-        if chain:
-            Fn.gemv_chain(phases, [True, True, True], bar)
-        else:
-            for ph in phases:
-                kw = dict(ph)
-                Fn.linear_decode(kw.pop("x"), kw.pop("w"), **kw)
-        torch.cuda.synchronize()
-        return x, h1, act, q
-
-    bar = torch.zeros(64, dtype=torch.int32, device=DEV)
-    want = run(False, kp_a, vp_a)
-    for _ in range(2):
-        got = run(True, kp_b, vp_b)
-        for g, w_, name in zip(got, want, ["x", "h1", "act", "q"]):
-            assert torch.equal(g, w_), f"{name} differs: max {((g.float() - w_.float()).abs().max().item())}"
-        assert torch.equal(kp_b, kp_a) and torch.equal(vp_b, vp_a)
-    assert int(bar[0].item()) == 0 and int(bar[32].item()) == 6  # {count, generation}: 3 barriers x 2 launches
-
-
-@pytest.mark.parametrize("M", [1, 2])
-def test_linear_decode_pipelined_main_loop_is_bit_identical(M):
-    """The software-pipelined main loop (two slot buffers, loads issued across task boundaries) keeps the accumulation order."""
-    torch.manual_seed(51)
-    # (shapes outside the split-K regime: that path sums in a different order)
-    cases = [(4096, 8192, {}), (8192, 1024, dict(residual=True)), (3584, 8192, dict(dual=True, norm=True)), (2050, 1032, {})]
-    for N, K, opt in cases:
-        x, w, w2 = _rand(M, K), _rand(N, K, scale=K ** -0.5), _rand(N, K, scale=K ** -0.5)
-        kw = {}
-        if opt.get("residual"):
-            kw["residual"] = _rand(M, N)
-        if opt.get("norm"):
-            kw.update(norm_weight=_rand(K) * 0.1 + 1, norm_kind=Fn.NORM_RMS, eps=1e-5)
-        if opt.get("dual"):
-            kw.update(w2=w2, act=Fn.ACT_SWIGLU)
-        try:
-            Fn.set_gemv_pipe(False)
-            want = Fn.linear_decode(x, w, **kw)
-            Fn.set_gemv_pipe(True)
-            got = Fn.linear_decode(x, w, **kw)
-        finally:
-            Fn.set_gemv_pipe(False)
-        assert torch.equal(got, want), f"N={N} K={K} {opt}: max diff {(got.float() - want.float()).abs().max().item()}"
-
-
 @pytest.mark.parametrize("M", [1, 4])
 def test_linear_decode_split_k_small_n(M):
     """Projections with few output columns (tensor-parallel QKV shards) run split-K inside the CTA: 4 warps share a row pair."""
